@@ -330,7 +330,27 @@ def flush_l2(torch, buf):
     buf.add_(1)   # 512 MB read+write > 126 MB L2
 
 
-def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=None):
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float64, so that two builds can be compared output for output.
+    When they would take more than DUMP_LIMIT_BYTES in all, every array of more than 1 MB is replaced by a fixed, seeded
+    sample of its rows, whose indices go to <name>_rows.npy (a row takes at least as many bytes as its index)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    large = sum(a.nbytes for a in arrays.values() if a.nbytes > (1 << 20))
+    small = sum(a.nbytes for a in arrays.values()) - large
+    for name, a in arrays.items():
+        if small + large > DUMP_LIMIT_BYTES and a.nbytes > (1 << 20):
+            keep = max(1, int(a.shape[0] * (DUMP_LIMIT_BYTES - small) / (2 * large)))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=None, dump_dir=None):
     from bundler_sfm_b200 import bundle, synth
     os.environ.setdefault("BSFM_BA_VERBOSE", "0")
     cfg = BA_CFGS[cfg_key]
@@ -352,7 +372,7 @@ def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         its, info = bundle.levmar_model(n, m, d_vmask.data_ptr(), d_p.data_ptr(), d_x.data_ptr(), cnp, R_init, f_fixed)
-        return its, time.perf_counter() - t0, bundle.last_timing()
+        return its, time.perf_counter() - t0, bundle.last_timing(), info
 
     vm_pin, _keep_vm = pinned_view(torch, scene["vmask"])
     pr_pin, _keep_pr = pinned_view(torch, scene["projections"])
@@ -379,10 +399,13 @@ def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=
         its_sum, dev_ms, wall = 0, 0.0, 0.0
         for _ in range(steps):
             flush_l2(torch, flush)
-            its, w, tm = solve_resident()
+            its, w, tm, info = solve_resident()
             its_sum += its; wall += w; dev_ms += tm["total_ms"]
         torch.cuda.synchronize()
         launches = lib.bsfm_kernel_launches() - launches0
+        if dump_dir is not None:     # the last timed solve: refined parameters (cameras, then points) and info[10]
+            p = d_p.cpu().numpy()
+            dumped = {"cameras": p[:m * cnp].reshape(m, cnp), "points": p[m * cnp:].reshape(n, 3), "info": info}
         if dist is not None:
             dist.barrier()
         e_its, e_wall = 0, 0.0
@@ -395,7 +418,7 @@ def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=
         # one more solve with per-phase events and (large systems) per-kernel-class events of the dense Cholesky
         os.environ["BSFM_BA_TIMING"] = "1"
         lib.bsfm_ba_chol_profile(1)
-        _, _, tm = solve_resident()
+        _, _, tm, _ = solve_resident()
         os.environ.pop("BSFM_BA_TIMING")
         pms = (ctypes.c_float * 4)(); pl = (ctypes.c_int * 4)(); ops = ctypes.c_double(); fl = ctypes.c_double()
         lib.bsfm_ba_chol_profile_read(pms, pl, ctypes.byref(ops), ctypes.byref(fl))
@@ -403,6 +426,8 @@ def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=
     finally:
         os.dup2(saved, 1)
         os.close(saved)
+    if dump_dir is not None:
+        dump_outputs(dump_dir, dumped)
     rmse = float(np.sqrt(out["info"][1] / nvis))
     # max over ranks (device-event time of the solves), sum of iterations
     t = torch.tensor([dev_ms * 1e-3, e_wall, float(its_sum), float(e_its)], dtype=torch.float64, device=dev)
@@ -438,7 +463,7 @@ def bench_ba(args, torch, dist, rank, world, dev, cfg_key, steps, warmup, scene=
     return res
 
 
-def bench_match(args, torch, dist, rank, world, dev, num_images, keys_per_image, steps, warmup):
+def bench_match(args, torch, dist, rank, world, dev, num_images, keys_per_image, steps, warmup, dump_dir=None):
     from bundler_sfm_b200 import keymatch, synth
     imgs = synth.sift_like_descriptors(num_images, keys_per_image, seed=7)
     keys, key_off = keymatch.concat_keys(imgs)
@@ -481,6 +506,9 @@ def bench_match(args, torch, dist, rank, world, dev, num_images, keys_per_image,
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = lib.bsfm_kernel_launches() - launches0
+    if dump_dir is not None and rank == 0:     # the table of the last timed pass (all ranks' shards when gathered)
+        c_last, m_last = db.fetch() if comm is None else db.gathered_fetch()
+        dump_outputs(dump_dir, {"pair_counts": c_last, "matches": m_last})
     if dist is not None:
         dist.barrier()
     # e2e: host descriptors (pinned) -> upload -> run -> gather -> table on the host
@@ -594,6 +622,8 @@ def main():
     ap.add_argument("--match-images", type=int, default=MATCH_CFG["num_images"])
     ap.add_argument("--no-side", action="store_true", help="skip the side objects (ba_config2 / match / ba_replicas)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the headline path computed in its last step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         return main_reference(args)
@@ -661,7 +691,8 @@ def main():
     if wl in ("ba2", "ba3"):
         from bundler_sfm_b200 import synth
         scene = synth.ba_scene(seed=1234 + rank, **BA_CFGS[wl])
-        ba = bench_ba(args, torch, dist, rank, world, dev, wl, steps=args.steps, warmup=args.warmup, scene=scene)
+        ba = bench_ba(args, torch, dist, rank, world, dev, wl, steps=args.steps, warmup=args.warmup, scene=scene,
+                      dump_dir=args.dump_outputs if rank == 0 else None)
         line = {"n_gpus": world, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "data": "synthetic", **ba_object(ba, wl)}
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             cpu = cpu_baseline_ba3(scene) if wl == "ba3" else cpu_baseline_ba2()
@@ -676,7 +707,8 @@ def main():
             line["match"] = match_object(m)
     else:
         # the headline of this workload: EXACTLY --steps timed passes behind --warmup (>= 3) untimed ones (a pass is 0.05-0.35 s)
-        m = bench_match(args, torch, dist, rank, world, dev, args.match_images, MATCH_CFG["keys_per_image"], steps=max(1, args.steps), warmup=args.warmup)
+        m = bench_match(args, torch, dist, rank, world, dev, args.match_images, MATCH_CFG["keys_per_image"], steps=max(1, args.steps), warmup=args.warmup,
+                        dump_dir=args.dump_outputs)
         line = {"n_gpus": world, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "data": "synthetic", **match_object(m)}
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             cpu = cpu_baseline_match()

@@ -1,6 +1,7 @@
 /* tests/c/sba_boundary_main.c -- boundary test of the sba-1.5 drop-in (shim/sba_b200.c).
- * Compiled against the REFERENCE's own lib/sba-1.5/sba.h (shim/Makefile: -I/root/reference/lib/sba-1.5), so the calls
- * below type-check against the reference declarations of sba_motstr_levmar / sba_mot_levmar (sba.h:96-115), and linked
+ * When the reference sources are at hand it is compiled against the REFERENCE's own lib/sba-1.5/sba.h (shim/Makefile,
+ * BSFM_REFERENCE_SBA_H), so the calls below type-check against the reference declarations of sba_motstr_levmar /
+ * sba_mot_levmar (sba.h:96-115); otherwise against the declarations below, which are those of shim/sba_b200.c.  Linked
  * against libsba_b200.so + libsfmdrv_b200.so instead of libsba.v1.5.a + libsfmdrv.a.
  *   sba_boundary_test <scene.bin> <result.bin> [mot]   solve the scene the way run_sfm does (sfm.c:652-838)
  *   sba_boundary_test foreign                          a foreign projection callback must fail loudly with SBA_ERROR
@@ -9,8 +10,28 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#ifdef BSFM_REFERENCE_SBA_H
 #include "sba.h"              /* the reference header */
+#endif
 #include "bsfm_b200_sba.h"    /* sfm_global_t mirror + the exported sfm_project_point3 */
+#ifndef BSFM_REFERENCE_SBA_H
+#define SBA_INFOSZ 10
+#define SBA_ERROR (-1)
+int sba_motstr_levmar(const int n, const int m, const int mcon, char *vmask, double *p, const int cnp, const int pnp,
+                      double *x, double *covx, const int mnp,
+                      void (*proj)(int j, int i, double *aj, double *bi, double *xij, void *adata),
+                      void (*projac)(int j, int i, double *aj, double *bi, double *Aij, double *Bij, void *adata),
+                      void *adata, const int itmax, const int verbose, const double *opts, double *info,
+                      int use_constraints, bsfm_camera_constraints_t *constraints,
+                      int use_point_constraints, bsfm_point_constraints_t *point_constraints,
+                      double *Vout, double *Sout, double *Uout, double *Wout);
+int sba_mot_levmar(const int n, const int m, const int mcon, char *vmask, double *p, const int cnp,
+                   double *x, double *covx, const int mnp,
+                   void (*proj)(int j, int i, double *aj, double *xij, void *adata),
+                   void (*projac)(int j, int i, double *aj, double *Aij, void *adata),
+                   void *adata, const int itmax, const int verbose, const double *opts, double *info,
+                   int use_constraints, bsfm_camera_constraints_t *constraints);
+#endif
 
 static void foreign_proj(int j, int i, double *aj, double *bi, double *xij, void *adata)
 {

@@ -149,8 +149,8 @@ def test_tc_equals_dp4a_at_scale(monkeypatch):
 
 def test_config4_table_sampled_pairs_vs_oracle_and_reference_exact(oracle):
     """BASELINE.json configs[3] at full size (500 images x 5000 keys, 124,750 pairs): 200 randomly drawn image pairs of the
-    GPU table are compared with the CPU oracle (pinned to the reference), and a handful of them with the UNMODIFIED
-    reference MatchKeys in exact mode (max_pts_visit = 0, keys2a.cpp:347-372) when oracle/_ref is present."""
+    GPU table are compared with the CPU oracle (pinned to the reference), and a handful of them with the stored output of the
+    UNMODIFIED reference MatchKeys in exact mode (max_pts_visit = 0, keys2a.cpp:347-372; tests/golden/reference_golden.npz)."""
     N, K = 500, 5000
     imgs = synth.sift_like_descriptors(N, K, seed=7)
     pairs, counts, matches = keymatch.key_match_full(imgs, -1, 0.6)
@@ -161,17 +161,20 @@ def test_config4_table_sampled_pairs_vs_oracle_and_reference_exact(oracle):
     # make sure rich pairs (consecutive images share 30 % noisy copies) are represented, not only sparse ones
     rich = [q for q, (j, i) in enumerate(pairs) if i == j + 1][::25]
     picked = np.unique(np.concatenate([picked, np.array(rich[:20], dtype=picked.dtype)]))
-    have_ref = oracle.ref_match() is not None
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_golden.npz"))
+    ref_pairs = [tuple(int(v) for v in p) for p in g["config4_pairs"]]
+    ref_starts = np.concatenate([[0], np.cumsum(g["config4_counts"])])
     nref = 0
     for q in picked:
         j, i = pairs[q]
         got = matches[starts[q]:starts[q + 1]]
         want = oracle.match_pair_port(imgs[j], imgs[i], 0.6)
         assert np.array_equal(got, want), (j, i)
-        if have_ref and (nref < 3 or (i == j + 1 and nref < 6)):
-            assert np.array_equal(got, oracle.match_pair_ref(imgs[j], imgs[i], 0.6, 0)), ("reference exact mode", j, i)
+        if nref < 3 or (i == j + 1 and nref < 6):
+            assert ref_pairs[nref] == (j, i)
+            assert np.array_equal(got, g["config4_matches"][ref_starts[nref]:ref_starts[nref + 1]]), ("reference exact mode", j, i)
             nref += 1
-    assert not have_ref or nref >= 3
+    assert nref == len(ref_pairs) >= 3
 
 
 def test_kermit_real_sift_table_equals_reference(kernel):

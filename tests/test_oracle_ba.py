@@ -1,7 +1,8 @@
 """CPU tests (no GPU): pin the BA oracle restatement (oracle/ba_oracle.c) against the committed outputs
 of the unmodified reference (tests/golden/ba_golden.npz, produced by tests/golden/make_ba_golden.py from
 lib/sba-1.5 + lib/sfm-driver compiled in place) and, when oracle/_ref is built, against the reference
-itself on a fresh scene.  Differences can only come from LAPACK's vs the restatement's Cholesky rounding."""
+itself on a fresh scene (stored in tests/golden/reference_golden.npz).  Differences can only come from LAPACK's vs the
+restatement's Cholesky rounding."""
 import os
 
 import numpy as np
@@ -10,6 +11,7 @@ import pytest
 from bundler_sfm_b200 import bundle, synth
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "ba_golden.npz")
+REF_GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_golden.npz")
 
 
 def rel(a, b):
@@ -49,13 +51,13 @@ def test_port_matches_reference_golden_constraints(oracle):
 
 
 def test_port_vs_reference_fresh(oracle):
-    if oracle.ref_sba() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference)")
+    """a scene outside ba_golden.npz, against the stored run_sfm results of the reference (tests/golden/make_reference_golden.py)"""
+    g = np.load(REF_GOLD)
     scene = synth.ba_scene(7, 250, 4, seed=31)
     pc = np.zeros_like(scene["pts"]); pc[::5] = scene["gt_pts"][::5]
-    for kw in ({}, {"ncons": 2}, dict(use_point_constraints=1, points_constraints=pc, point_constraint_weight=0.3)):
+    for q, kw in enumerate(({}, {"ncons": 2}, dict(use_point_constraints=1, points_constraints=pc, point_constraint_weight=0.3))):
         got = oracle.run_sfm_port(scene, **kw)
-        ref = oracle.run_sfm_ref(scene, **kw)
+        ref = {k: g[f"bafresh{q}_{k}"] for k in ("R", "c", "f", "k", "pts", "info")}
         check(got, ref, scene["projections"].shape[0], str(kw))
 
 

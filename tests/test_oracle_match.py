@@ -1,6 +1,6 @@
 """CPU tests (no GPU): pin the MATCH oracle restatement (oracle/match_oracle.c) against the golden
-vectors produced by the unmodified reference (tests/golden/make_match_golden.py) and, when
-oracle/_ref is built, against the reference itself on fresh random inputs."""
+vectors produced by the unmodified reference (tests/golden/make_match_golden.py) and against its stored results on further
+inputs (tests/golden/make_reference_golden.py)."""
 import os
 
 import numpy as np
@@ -9,11 +9,17 @@ import pytest
 from bundler_sfm_b200 import synth
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "match_golden.npz")
+REF_GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_golden.npz")
 
 
 @pytest.fixture(scope="module")
 def gold():
     return np.load(GOLD)
+
+
+@pytest.fixture(scope="module")
+def ref_gold():
+    return np.load(REF_GOLD)
 
 
 def test_port_matches_golden_sift_pairs(oracle, gold):
@@ -58,16 +64,13 @@ def test_cap200_recall_informational(gold):
     assert tot > 0 and hit / tot > 0.5
 
 
-def test_port_vs_reference_random(oracle):
-    if oracle.ref_match() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference)")
+def test_port_vs_reference_random(oracle, ref_gold):
     for seed in range(3):
         imgs = synth.sift_like_descriptors(2, [300 + 17 * seed, 280], seed=100 + seed)
         a = oracle.match_pair_port(imgs[0], imgs[1], 0.6)
-        b = oracle.match_pair_ref(imgs[0], imgs[1], 0.6, 0)
-        assert np.array_equal(a, b)
+        assert np.array_equal(a, ref_gold[f"matchrnd{seed}_sift"])
         u1, u2 = synth.random_descriptors(90, seed), synth.random_descriptors(75, seed + 50)
-        assert np.array_equal(oracle.match_pair_port(u1, u2, 0.95), oracle.match_pair_ref(u1, u2, 0.95, 0))
+        assert np.array_equal(oracle.match_pair_port(u1, u2, 0.95), ref_gold[f"matchrnd{seed}_uniform"])
 
 
 def test_all_pairs_table_format(oracle):
@@ -91,16 +94,14 @@ def test_all_pairs_table_format(oracle):
     assert counts_w[3, 0] == 0 and counts_w[3, 2] == counts[3, 2]
 
 
-def test_port_keys_cpp_test_mode_vs_reference_exhaustive():
-    """oracle/match_oracle.c mode 1 (sqrt(d0/d1) <= ratio, `registered` subset) against the UNMODIFIED MatchKeysExhaustive of
-    src/keys.cpp (oracle/_ref/libref_keys.so): the pair of calls bundler --add_images makes (Bundle.cpp:3812-3820)"""
+def test_port_keys_cpp_test_mode_vs_reference_exhaustive(ref_gold):
+    """oracle/match_oracle.c mode 1 (sqrt(d0/d1) <= ratio, `registered` subset) against the stored results of the UNMODIFIED
+    MatchKeysExhaustive of src/keys.cpp: the pair of calls bundler --add_images makes (Bundle.cpp:3812-3820)"""
     from oracle import loader
-    if loader.ref_keys() is None:
-        pytest.skip("oracle/_ref/libref_keys.so not built")
     imgs = synth.sift_like_descriptors(2, [600, 750], seed=11)
     extra = np.where(np.random.default_rng(3).random(750) < 0.6, 5, -1).astype(np.int32)
-    for reg, ratio in ((True, 0.75), (False, 1.0), (False, 0.6), (True, 0.9)):
-        want = loader.keys_match_ref(imgs[0], imgs[1], extra, reg, ratio, exhaustive=True)
+    for q, (reg, ratio) in enumerate(((True, 0.75), (False, 1.0), (False, 0.6), (True, 0.9))):
+        want = ref_gold[f"keyscpp{q}_matches"]
         got = loader.match_pair_port_test(imgs[0], imgs[1], ratio, 1, extra, reg)
         assert np.array_equal(got, want), (reg, ratio)
         assert want.shape[0] > 0

@@ -3,6 +3,7 @@ solver, and the UNMODIFIED reference KeyMatchFull main (src/KeyMatchFull.cpp) li
 MatchKeys shim.  The CPU tests only check the artefacts exist and export the reference symbols; the GPU
 tests run them."""
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -17,7 +18,8 @@ KM = os.path.join(BUILD, "KeyMatchFull_b200")
 KMP = os.path.join(BUILD, "KeyMatchFull_b200_persistent")
 KEYFILE = os.path.join(BUILD, "libkeyfile_b200.so")
 SFMDRV = os.path.join(BUILD, "libsfmdrv_b200.so")
-REFMATCH = os.path.join(ROOT, "oracle", "_ref", "libref_match.so")
+# what the unmodified reference returned on the inputs of these tests (tests/golden/make_reference_golden.py)
+REF_GOLD = os.path.join(ROOT, "tests", "golden", "reference_golden.npz")
 
 
 def test_sfmdrv_shim_exports_run_sfm():
@@ -29,9 +31,14 @@ def test_sfmdrv_shim_exports_run_sfm():
 
 def test_keymatchfull_shim_binary_links_reference_main():
     if not os.path.exists(KM):
-        pytest.skip("shim/_build/KeyMatchFull_b200 not built (needs /root/reference at build time)")
+        pytest.skip("shim/_build/KeyMatchFull_b200 not built (needs the reference sources at build time)")
     r = subprocess.run([KM], capture_output=True, text=True)
     assert "Usage:" in r.stdout and "<list.txt> <outfile> [window_radius]" in r.stdout   # KeyMatchFull.cpp:65
+
+
+def _sha256(a):
+    """digest under which tests/golden/make_reference_golden.py stores the descriptor lists the reference read"""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def _read_with(fn, path):
@@ -45,34 +52,33 @@ def _read_with(fn, path):
 
 
 def test_key_reader_equals_reference_readkeyfile(tmp_path):
-    """shim/keyfile_b200.cpp against the unmodified reference parser (src/keys2a.cpp:87-323 compiled in
-    oracle/_ref): plain file, gzip fallback, empty image, missing file, bad descriptor length."""
-    if not (os.path.exists(KEYFILE) and os.path.exists(REFMATCH)):
-        pytest.skip("shim/_build or oracle/_ref not built")
+    """shim/keyfile_b200.cpp against the stored results of the unmodified reference parser (src/keys2a.cpp:87-323) on the
+    same files: plain file, gzip fallback, empty image, missing file, bad descriptor length."""
+    if not os.path.exists(KEYFILE):
+        pytest.skip("shim/_build not built")
     import gzip
+    g = np.load(REF_GOLD)
+    ref_n, ref_sha = g["keyfile_n"], g["keyfile_sha256"]
     ours = ctypes.CDLL(KEYFILE).bsfm_shim_read_key_file
-    ref = getattr(ctypes.CDLL(REFMATCH), "_Z11ReadKeyFilePKcPPhPP7keypt_t")
     imgs = synth.sift_like_descriptors(3, [257, 1, 40], seed=5)
     for i, d in enumerate(imgs):
         p = str(tmp_path / f"a{i}.key")
         synth.write_key_file(p, d, seed=i)
-        n0, k0 = _read_with(ref, p)
         n1, k1 = _read_with(ours, p)
-        assert n0 == n1 == d.shape[0] and np.array_equal(k0, k1) and np.array_equal(k1, d)
+        assert ref_n[i] == n1 == d.shape[0] and _sha256(k1) == ref_sha[i] and np.array_equal(k1, d)
     # gzip fallback: only <name>.gz exists (keys2a.cpp:93-104)
     p = str(tmp_path / "z.key")
     synth.write_key_file(p, imgs[0], seed=9)
-    with open(p, "rb") as f, gzip.open(p + ".gz", "wb") as g:
-        g.write(f.read())
+    with open(p, "rb") as f, gzip.open(p + ".gz", "wb") as gz:
+        gz.write(f.read())
     os.remove(p)
-    n0, k0 = _read_with(ref, p)
     n1, k1 = _read_with(ours, p)
-    assert n0 == n1 == 257 and np.array_equal(k0, k1)
+    assert ref_n[3] == n1 == 257 and _sha256(k1) == ref_sha[3]
     # empty image, missing file, wrong descriptor length: both return 0
     (tmp_path / "e.key").write_text("0 128\n")
     (tmp_path / "bad.key").write_text("1 64\n" + "1 2 3 4\n" + " ".join(["7"] * 64) + "\n")
-    for name in ("e.key", "missing.key", "bad.key"):
-        assert _read_with(ref, str(tmp_path / name))[0] == 0
+    for q, name in enumerate(("e.key", "missing.key", "bad.key")):
+        assert ref_n[4 + q] == 0
         assert _read_with(ours, str(tmp_path / name))[0] == 0
 
 
@@ -189,19 +195,24 @@ def _read_result(path, scene, cnp):
     return rc, info, p
 
 
+def _gold_ref(prefix, keys=("R", "c", "f", "k", "pts", "info")):
+    g = np.load(REF_GOLD)
+    return {k: g[f"{prefix}_{k}"] for k in keys}
+
+
 @pytest.mark.gpu
-def test_sba_motstr_levmar_reference_signature_program(tmp_path, oracle):
+def test_sba_motstr_levmar_reference_signature_program(tmp_path):
     from bundler_sfm_b200 import bundle
     exe = os.path.join(BUILD, "sba_boundary_test")
     if not os.path.exists(exe):
-        pytest.skip("shim/_build/sba_boundary_test not built (needs /root/reference headers at build time)")
+        pytest.skip("shim/_build/sba_boundary_test not built")
     scene = synth.ba_scene(12, 700, 4, seed=77)
     nvis = scene["projections"].shape[0]
     _write_scene(tmp_path / "scene.bin", scene)
     r = subprocess.run([exe, str(tmp_path / "scene.bin"), str(tmp_path / "res.bin")], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
     rc, info, p = _read_result(tmp_path / "res.bin", scene, 9)
-    ref = oracle.run_sfm_oracle(scene)
+    ref = _gold_ref("motstr")                # run_sfm of the unmodified reference on this scene
     assert rc == int(ref["info"][5]) == int(info[5])                    # returns the iteration count like the reference
     assert int(info[6]) == int(ref["info"][6])
     assert abs(np.sqrt(info[1] / nvis) - np.sqrt(ref["info"][1] / nvis)) <= 1e-5
@@ -216,10 +227,10 @@ def test_sba_motstr_levmar_reference_signature_program(tmp_path, oracle):
 
 
 @pytest.mark.gpu
-def test_sba_mot_levmar_reference_signature_program(tmp_path, oracle):
+def test_sba_mot_levmar_reference_signature_program(tmp_path):
     exe = os.path.join(BUILD, "sba_boundary_test")
-    if not os.path.exists(exe) or oracle.ref_sba() is None:
-        pytest.skip("needs shim/_build/sba_boundary_test and oracle/_ref")
+    if not os.path.exists(exe):
+        pytest.skip("shim/_build/sba_boundary_test not built")
     from bundler_sfm_b200 import bundle
     scene = synth.ba_scene(10, 500, 4, seed=78)
     nvis = scene["projections"].shape[0]
@@ -227,7 +238,7 @@ def test_sba_mot_levmar_reference_signature_program(tmp_path, oracle):
     r = subprocess.run([exe, str(tmp_path / "scene.bin"), str(tmp_path / "res.bin"), "mot"], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
     rc, info, p = _read_result(tmp_path / "res.bin", scene, 9)
-    ref = oracle.run_sfm_ref(scene, fix_points=1)
+    ref = _gold_ref("mot", ("R", "c", "f", "k", "info"))      # run_sfm(fix_points = 1) of the unmodified reference
     assert abs(rc - int(ref["info"][5])) <= 3 and int(info[6]) in (2, 4)     # eps4 = 0 knife-edge, see test_ba_gpu.check_mot_solution
     assert abs(np.sqrt(info[1] / nvis) - np.sqrt(ref["info"][1] / nvis)) <= 1e-5
     got = bundle.unpack_params(p, scene)
@@ -297,7 +308,7 @@ def test_match_pair_test_modes_vs_port(oracle):
 
 def test_binary_key_cache_roundtrip_and_reference_reader(tmp_path):
     """<name>.bin in the layout of src/keys.cpp:551-648: written from a parsed text file, read back when the text file is gone,
-    and accepted by the UNMODIFIED in-bundler reader ReadKeyFileWithDesc (oracle/_ref/libref_keys.so)"""
+    and byte for byte the file the UNMODIFIED in-bundler reader ReadKeyFileWithDesc was run on (stored with what it read)"""
     if not os.path.exists(KEYFILE):
         pytest.skip("shim/_build not built")
     lib = ctypes.CDLL(KEYFILE)
@@ -318,11 +329,7 @@ def test_binary_key_cache_roundtrip_and_reference_reader(tmp_path):
     assert rd(txt.encode(), ctypes.byref(kbuf2), ctypes.byref(ibuf2)) == n
     assert np.array_equal(np.ctypeslib.as_array(kbuf2, shape=(n * 128,)).reshape(n, 128), d)
     assert np.array_equal(np.ctypeslib.as_array(ibuf2, shape=(n * 4,)).reshape(n, 4), info)
-    refso = os.path.join(ROOT, "oracle", "_ref", "libref_keys.so")
-    if os.path.exists(refso):                        # the reference's own reader on the file we wrote
-        ref = ctypes.CDLL(refso)
-        fn = ref.ref_read_key_file_with_desc
-        fn.restype = ctypes.c_int
-        out = np.zeros((n, 128), np.uint8); xy = np.zeros((n, 2), np.float32)
-        assert fn(txt.encode(), out.ctypes.data_as(ctypes.c_void_p), xy.ctypes.data_as(ctypes.c_void_p), n) == n
-        assert np.array_equal(out, d) and np.array_equal(xy, info[:, :2])
+    g = np.load(REF_GOLD)                            # the reference's own reader on the file written by the same code
+    assert hashlib.sha256(open(txt + ".bin", "rb").read()).hexdigest() == g["keybin_file_sha256"]
+    assert g["keybin_ref_n"] == n
+    assert g["keybin_ref_desc_sha256"] == _sha256(d) and np.array_equal(g["keybin_ref_xy"], info[:, :2])
